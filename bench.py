@@ -485,6 +485,7 @@ class Bench:
         self.extrap = pysteps_b200.extrapolation.get_method("semilagrangian")
         self.lk = have_lk()
         self.flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device="cuda")  # > 126 MB L2
+        self.last_out = None
 
     def motion(self, name):
         if not self.lk:
@@ -511,11 +512,13 @@ class Bench:
         self.dist.broadcast(t, src=0)
         return bool(t.item())
 
-    def time_device(self, step, steps, warmup, min_warm_s=0.0, marks=None, sampler=None):
+    def time_device(self, step, steps, warmup, min_warm_s=0.0, marks=None, sampler=None, keep_last=False):
         """W >= 3 untimed steps (stretched to min_warm_s of the same load for the clock sampler),
         then `steps` steps, each bracketed by barrier + synchronize and CUDA events, L2 flushed in
         between (outside the events).  Returns (ms summed over steps [max over ranks], trace,
-        launches, per-phase ms when the step records `marks`)."""
+        launches, per-phase ms when the step records `marks`).  keep_last: the last timed step's
+        result is left in self.last_out (earlier results are dropped as they come, so the allocator
+        sees the same pattern as without it)."""
         torch = self.torch
         t_w, n_w = time.perf_counter(), 0
         while True:
@@ -543,7 +546,10 @@ class Bench:
                 self.flush.fill_(1)
                 self.barrier()
                 s.record()
-                step()
+                if keep_last and i == steps - 1:
+                    self.last_out = step()
+                else:
+                    step()
                 e.record()
                 if marks is not None:
                     phase.append(list(marks))
@@ -790,8 +796,44 @@ FP64_PER_CLK_SM = 64
 SL_FP64_INSTR_PER_PIXEL_LEADTIME = 94
 
 
-def measure(b, w, steps, warmup, clocks=None, solo=False):
-    """device-resident + end-to-end timing of one workload -> dict (rank 0) / None."""
+DUMP_LIMIT = 64 * 10 ** 6  # bytes written by --dump-outputs, all files together
+# what --dump-outputs writes for a pixel the extrapolation leaves undefined (outval=nan: advected in from
+# outside the domain).  The dumped fields are precipitation (>= 0), so the value cannot be a real one.
+DUMP_UNDEFINED = -9999.0
+
+
+def dump_outputs(out, dirpath):
+    """Writes what one step of the timed path returned as DIR/<name>.npy (float32 / float64).  An
+    array larger than its share of DUMP_LIMIT is cut to a fixed, seeded sample of rows (axis -2),
+    the same rows on every run, so that two builds can be compared output for output.  The files hold
+    finite numbers only: NaN is written as DUMP_UNDEFINED, which a dumped field never holds otherwise
+    (checked here, as is the absence of infinities)."""
+    arrays = list(out) if isinstance(out, (tuple, list)) else [out]
+    names = ["extrapolated"] if len(arrays) == 1 else [f"extrapolated_{i}" for i in range(len(arrays))]
+    budget = DUMP_LIMIT // len(arrays) - 4096  # room for the .npy header
+    os.makedirs(dirpath, exist_ok=True)
+    written = {}
+    for name, a in zip(names, arrays):
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        shape = list(a.shape)
+        if a.nbytes > budget:
+            rows = a.shape[-2]
+            keep = max(1, budget * rows // a.nbytes)
+            a = a[..., np.sort(np.random.default_rng(0).choice(rows, keep, replace=False)), :]
+        nan = np.isnan(a)
+        if np.isinf(a).any() or (a == DUMP_UNDEFINED).any():
+            raise ValueError(f"--dump-outputs: {name} holds an infinity or the value {DUMP_UNDEFINED}")
+        np.save(os.path.join(dirpath, name + ".npy"), np.ascontiguousarray(np.where(nan, a.dtype.type(DUMP_UNDEFINED), a)))
+        written[name] = {"shape": shape, "saved_shape": list(a.shape), "dtype": str(a.dtype),
+                         "undefined_written_as": DUMP_UNDEFINED, "undefined": int(np.count_nonzero(nan))}
+    return written
+
+
+def measure(b, w, steps, warmup, clocks=None, solo=False, dump=None):
+    """device-resident + end-to-end timing of one workload -> dict (rank 0) / None.  dump: directory
+    that receives the last timed step's result (dump_outputs)."""
     if w["members"]:
         step_device, step_host, info = build_ensemble(b, w, solo=solo)
     else:
@@ -801,10 +843,15 @@ def measure(b, w, steps, warmup, clocks=None, solo=False):
     if clocks is not None:
         clocks.__enter__()
     dev_ms, tr, launches, phases = b.time_device(step_device, steps, warmup, 0.5 if clocks is not None else 0.0, marks,
-                                                 sampler=clocks)
+                                                 sampler=clocks, keep_last=dump is not None)
     each_ms = list(b.each_ms)
     if clocks is not None:
         clocks.__exit__(None, None, None)
+    dumped = None
+    if dump is not None:
+        if b.rank == 0 and b.last_out is not None:
+            dumped = dump_outputs(b.last_out, dump)
+        b.last_out = None
     nfields = info["nfields"]
     value = nfields * steps * T * m * n / (dev_ms * 1e-3) / 1e6
     stage_trace, stage_steps = b.stage_trace, b.stage_steps
@@ -841,6 +888,8 @@ def measure(b, w, steps, warmup, clocks=None, solo=False):
         blk["batched_note"] = ("extrapolate_members / b200_sl_step_batched (all members of a rank in one launch "
                                "per lead time): not a call the unmodified nowcast_main_loop makes; `value` is "
                                "the per-member call shape")
+    if dumped is not None:
+        blk["dumped_outputs"] = dumped
     return blk
 
 
@@ -940,7 +989,7 @@ def run_ours(args, w):
     b = Bench()
     peaks = load_peaks()
     clocks = ClockSampler(b.local, enabled=(b.rank == 0))
-    head = measure(b, w, args.steps, args.warmup, clocks=clocks)
+    head = measure(b, w, args.steps, args.warmup, clocks=clocks, dump=args.dump_outputs)
     extras = {}
     if not args.no_extras and args.workload == "lk_sl12_2048":
         for name in EXTRAS:
@@ -1010,7 +1059,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline workload only")
     ap.add_argument("--extra-steps", type=int, default=5, help="timed steps of the ensemble24 / composite4096 blocks")
     ap.add_argument("--workload", default="lk_sl12_2048", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's last timed step's result to DIR/<name>.npy, NaN as -9999 "
+                         "(at most 64 MB, a fixed seeded sample of rows beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = set_workload(args.workload)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":

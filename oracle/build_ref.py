@@ -15,6 +15,7 @@ sources where they lie -- no source file is copied:
 imported under a stub namespace package (oracle/refimport.py), which runs each submodule's own
 code unchanged.
 """
+import importlib.util
 import os
 import py_compile
 import shutil
@@ -79,8 +80,14 @@ def build():
     if not available():
         return False
     n = compile_modules()
-    for ext in ("_vet", "_proesmans"):
-        build_extension(ext)
+    if importlib.util.find_spec("Cython") is None:
+        # the bytecode alone serves the pure-Python modules; vet / proesmans of the reference and
+        # the tests that run its nowcast loop then skip
+        print("oracle/build_ref.py: Cython is not installed; the reference's _vet / _proesmans extensions "
+              "are not built")
+    else:
+        for ext in ("_vet", "_proesmans"):
+            build_extension(ext)
     with open(os.path.join(OUT, "README"), "w") as f:
         f.write("Built by oracle/build_ref.py from /root/reference (pysteps v1.21.3): bytecode of the package "
                 f"({n} modules) and its two Cython extensions.  Test infrastructure; not product code.\n")

@@ -61,3 +61,10 @@ def assert_bits_equal(a, b, what=""):
 def golden_sl():
     path = os.path.join(ROOT, "tests", "golden", "sl_golden.npz")
     return np.load(path)
+
+
+@pytest.fixture(scope="session")
+def reference_golden():
+    """outputs of pysteps v1.21.3 on tests/golden/reference_cases.py (gen_reference_golden.py)"""
+    import fingerprint
+    return fingerprint.load(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))

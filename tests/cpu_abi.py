@@ -544,6 +544,20 @@ def emulated():
         st.enter_context(mock.patch.object(torch.cuda, "current_device", lambda: 0))
         _side.clear()
         st.enter_context(mock.patch.object(torch.cuda, "current_stream", lambda *a: _Stream()))
+        # the module-level caches of streams, buffers and uploaded arrays get private, empty stand-ins:
+        # on a machine with a GPU, a real stream cached by an earlier test would otherwise meet the
+        # emulated events, and a host tensor cached here would later reach a real kernel as a pointer
+        import threading
+        from pysteps_b200.extrapolation import semilagrangian
+        from pysteps_b200.motion import lucaskanade
+        from pysteps_b200.noise import motion as noise_motion
+        st.enter_context(mock.patch.object(lucaskanade, "_side_streams", {}))
+        st.enter_context(mock.patch.object(lucaskanade, "_grids", {}))
+        st.enter_context(mock.patch.object(lucaskanade, "_readback", threading.local()))
+        st.enter_context(mock.patch.object(_device, "_recent", {}))
+        st.enter_context(mock.patch.object(semilagrangian, "_pinned", threading.local()))
+        st.enter_context(mock.patch.object(semilagrangian, "_default_grid_seen", {}))
+        st.enter_context(mock.patch.object(noise_motion, "_fields", {}))
         # a device tensor's .cpu() is a fresh host copy; keep that property for the stand-ins
         st.enter_context(mock.patch.object(torch.Tensor, "cpu", lambda self, *a, **k: self.clone()))
         yield

@@ -2,8 +2,9 @@
 plumbing, frame pairing and pooling, early-outs, masked-array handling, return conventions, the
 b200_rows extension) over randomised frames and argument combinations.  The C-ABI entry points are
 emulated with the oracle's stage functions (tests/cpu_abi.py), so the shim must reproduce the
-oracle's dense_lucaskanade -- itself pinned to the reference -- bit for bit; errors are compared
-with the live reference when /root/reference exists."""
+oracle's dense_lucaskanade -- itself pinned to the reference -- bit for bit; errors, sparse
+vectors and dense fields are also compared with the reference's stored outputs on the same calls
+(tests/golden/reference_lk_host_golden.npz, tests/golden/gen_reference_golden.py)."""
 import os
 import warnings
 
@@ -11,19 +12,18 @@ import numpy as np
 import pytest
 
 import cpu_abi
+import fingerprint as fp
 from oracle import lucaskanade as ora
 from pysteps_b200 import _synthetic as syn
 
 
-def _live():
-    from _refimport import available, ref_module
-    if not available():
-        return None
-    try:
-        import cv2  # noqa: F401
-    except ImportError:
-        return None
-    return ref_module("pysteps.motion.lucaskanade").dense_lucaskanade
+@pytest.fixture(scope="module")
+def golden():
+    return fp.load(os.path.join(os.path.dirname(__file__), "golden", "reference_lk_host_golden.npz"))
+
+
+def _error_entry(err):
+    return "" if err is None else "%s: %s" % err
 
 
 def _random_call(rng):
@@ -76,9 +76,8 @@ def _run(fn, inp, kw):
 
 
 @pytest.mark.parametrize("seed", range(4))
-def test_dense_lucaskanade_host_logic(seed):
+def test_dense_lucaskanade_host_logic(seed, golden):
     from pysteps_b200.motion.lucaskanade import dense_lucaskanade
-    live = _live()
     rng = np.random.default_rng(500 + seed)
     n_ok = n_err = n_empty = 0
     with cpu_abi.emulated():
@@ -88,9 +87,7 @@ def test_dense_lucaskanade_host_logic(seed):
             want, werr = _run(ora.dense_lucaskanade, inp, kw)
             ctx = f"seed {seed} case {it}: shape={inp.shape} masked={isinstance(inp, np.ma.MaskedArray)} kw={kw}"
             assert gerr == werr, ctx
-            if live is not None:
-                _, rerr = _run(live, inp, kw)
-                assert gerr == rerr, ctx
+            assert _error_entry(gerr) == str(golden[f"host/{seed}/{it}/error"]), ctx
             if gerr is not None:
                 n_err += 1
                 continue
@@ -140,13 +137,12 @@ def test_row_band_fill_and_stage_mirrors():
         assert np.array_equal(stages.idwinterp2d(dxy, duv, np.arange(96), np.arange(30, 70)), g[:, 30:70])
 
 
-def test_sparse_vectors_equal_the_live_reference():
+def test_sparse_vectors_equal_the_live_reference(golden):
     """The outlier stage takes neighbours in cKDTree's own order (csrc/knn.cu; emulated here by the
     kernel body compiled for the host): the sparse vectors equal the LIVE reference bit for bit --
     also on three-frame inputs whose pooled vectors coincide, where a lower-index rule would keep
     or drop a different vector (DESIGN.md section 4)."""
     from pysteps_b200.motion.lucaskanade import dense_lucaskanade
-    live = _live()
     rng = np.random.default_rng(2000)
     n = 0
     with cpu_abi.emulated():
@@ -157,24 +153,22 @@ def test_sparse_vectors_equal_the_live_reference():
             with ora.knn_mode("ckdtree"):
                 want, werr = _run(ora.dense_lucaskanade, inp, kw)
             assert gerr == werr, (it, kw)
+            assert _error_entry(gerr) == str(golden[f"sparse/{it}/error"]), (it, kw)
             if gerr is None:
                 n += 1
                 for a, b in zip(got, want):
                     assert a.shape == b.shape and np.array_equal(a, b), (it, kw)
-                if live is not None:
-                    ref, _ = _run(live, inp, kw)
-                    for a, b in zip(got, ref):
-                        assert a.shape == b.shape and np.array_equal(a, b), (it, kw)
+                fp.assert_same(got[0], golden, f"sparse/{it}/xy", f"{it} {kw}")
+                fp.assert_same(got[1], golden, f"sparse/{it}/uv", f"{it} {kw}")
     assert n >= 40
 
 
-def test_dense_field_equals_the_live_reference_everywhere():
-    """... and the dense field equals the live reference at EVERY pixel to the last bits, pixels
-    with a k-NN tie included."""
+def test_dense_field_equals_the_live_reference_everywhere(golden):
+    """... and the dense field equals the reference to the last bits (1e-13), pixels with a k-NN tie
+    included: bit for bit against the stored digest of the reference's field or, failing that, on its
+    stored sample, and at every pixel against the oracle in cKDTree mode (pinned to the reference by
+    tests/test_oracle_lk.py)."""
     from pysteps_b200.motion.lucaskanade import dense_lucaskanade
-    live = _live()
-    if live is None:
-        pytest.skip("/root/reference or cv2 not present")
     rng = np.random.default_rng(2001)
     n = 0
     with cpu_abi.emulated():
@@ -182,21 +176,22 @@ def test_dense_field_equals_the_live_reference_everywhere():
             inp, kw = _random_call(rng)
             kw = dict(kw, dense=True)
             got, gerr = _run(dense_lucaskanade, inp, kw)
-            ref, rerr = _run(live, inp, kw)
-            assert gerr == rerr, (it, kw)
+            assert _error_entry(gerr) == str(golden[f"dense/{it}/error"]), (it, kw)
             if gerr is None:
                 n += 1
-                assert got.shape == ref.shape and np.abs(got - ref).max() <= 1e-13, (it, kw)
+                fp.assert_close(got, golden, f"dense/{it}/field", 1e-13, f"case {it} {kw}")
+                with ora.knn_mode("ckdtree"):
+                    want = ora.dense_lucaskanade(inp.copy(), **kw)
+                assert np.abs(got - want).max() <= 1e-13, (it, kw)
     assert n >= 20
 
 
-def test_float32_frames_are_scaled_in_float32_like_the_reference():
+def test_float32_frames_are_scaled_in_float32_like_the_reference(golden):
     """float32 frames: NumPy scales them to uint8 in float32, which moves some pixels by one grey
     level against float64 arithmetic and with them corners and vectors; the shim flags the frames
-    (B200_QUANTISE_F32) and reproduces the oracle -- and, with the reference's tie order, the live
-    reference's sparse vectors."""
+    (B200_QUANTISE_F32) and reproduces the oracle -- and, with the reference's tie order, the
+    reference's stored sparse vectors."""
     from pysteps_b200.motion.lucaskanade import dense_lucaskanade
-    live = _live()
     rng = np.random.default_rng(0)
     with cpu_abi.emulated():
         for it in range(12):
@@ -211,9 +206,8 @@ def test_float32_frames_are_scaled_in_float32_like_the_reference():
             assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), it
             V = dense_lucaskanade(inp.copy())
             assert V.dtype == np.float64 and np.array_equal(V, ora.dense_lucaskanade(inp.copy())), it
-            if live is not None:
-                ref = live(inp.copy(), dense=False)
-                assert np.array_equal(got[0], ref[0]) and np.array_equal(got[1], ref[1]), it
+            fp.assert_same(got[0], golden, f"float32/{it}/xy", str(it))
+            fp.assert_same(got[1], golden, f"float32/{it}/uv", str(it))
 
 
 def test_many_frames_pool_larger_than_the_decluster_kernel(monkeypatch):

@@ -1,24 +1,26 @@
 """CPU test of the HOST logic of pysteps_b200.extrapolation.semilagrangian.extrapolate and of the
 BPS handles: argument validation (order, types, messages), defaults, return structure, dtypes
-and shapes, over randomised valid AND invalid argument combinations -- against the live
-reference when /root/reference exists, else against the oracle.  The C ABI is emulated by the
-oracle (tests/cpu_abi.py), so numerics here say nothing about the kernels."""
+and shapes, over randomised valid AND invalid argument combinations -- against the oracle and
+the reference's stored results on the same calls (tests/golden/reference_host_golden.npz, written
+by tests/golden/gen_reference_golden.py).  The C ABI is emulated by the oracle (tests/cpu_abi.py),
+so numerics here say nothing about the kernels."""
+import os
 import warnings
 
 import numpy as np
 import pytest
 
 import cpu_abi
+import fingerprint as fp
+import reference_cases as rc
 from oracle import noise_motion as ora_bps
 from oracle import semilagrangian as ora
 from pysteps_b200 import _synthetic as syn
 
 
-def _reference():
-    from _refimport import available, ref_module
-    if available():
-        return ref_module("pysteps.extrapolation.semilagrangian").extrapolate, True
-    return ora.extrapolate, False
+@pytest.fixture(scope="module")
+def golden():
+    return fp.load(os.path.join(os.path.dirname(__file__), "golden", "reference_host_golden.npz"))
 
 
 def _bits_equal(a, b):
@@ -104,17 +106,18 @@ def _run(fn, Pin, Vin, ts, outval, kw):
 
 
 @pytest.mark.parametrize("seed", range(6))
-def test_extrapolate_host_logic_matches_reference(seed):
+def test_extrapolate_host_logic_matches_reference(seed, golden):
     import pysteps_b200
-    ref, live = _reference()
     rng = np.random.default_rng(100 + seed)
     n_err = n_ok = 0
     with cpu_abi.emulated():
         for it in range(120):
             Pin, Vin, ts, outval, kw = _random_call(rng)
-            want, werr, wdep = _run(ref, Pin, Vin, ts, outval, kw)
+            want, werr, wdep = _run(ora.extrapolate, Pin, Vin, ts, outval, kw)
             got, gerr, gdep = _run(pysteps_b200.extrapolation.semilagrangian.extrapolate, Pin, Vin, ts, outval, kw)
             ctx = f"seed {seed} case {it}: ts={ts!r} outval={outval!r} kw={ {k: (v.shape if isinstance(v, np.ndarray) else v) for k, v in kw.items()} }"
+            fp.assert_call(got, gerr, golden, f"sl/{seed}/{it}", ctx)
+            assert "\n".join(gdep) == golden[f"sl/{seed}/{it}/deprecations"], ctx
             assert gerr == werr, ctx
             assert gdep == wdep, ctx
             if werr is not None:
@@ -126,37 +129,34 @@ def test_extrapolate_host_logic_matches_reference(seed):
                 assert (a is None) == (b is None), ctx
                 if a is not None:
                     assert isinstance(a, np.ndarray) and _bits_equal(a, b), ctx
-    assert n_err >= 10 and n_ok >= 40, (n_err, n_ok, live)
+    assert n_err >= 10 and n_ok >= 40, (n_err, n_ok)
 
 
-def test_member_loop_with_handles_matches_reference_expression():
+def test_member_loop_with_handles_matches_reference_expression(golden):
     """nowcasts/utils.py:440-458 with lazy handles and resident displacements == the same loop
-    with materialised arrays (oracle perturbator + the reference / oracle extrapolator)."""
+    with materialised arrays (oracle perturbator + oracle extrapolator, whose results equal the
+    reference's stored ones)."""
     import pysteps_b200
     from pysteps_b200 import _device
-    ref, _ = _reference()
-    rng = np.random.default_rng(5)
     with cpu_abi.emulated():
         init, gen = pysteps_b200.noise.get_method("bps")
         extrap = pysteps_b200.extrapolation.get_method("semilagrangian")
-        for vd in (np.float64, np.float32):
-            V = (3 * rng.standard_normal((2, 19, 23))).astype(vd)
-            V[:, 4:7, 5:9] = 0
-            P = rng.standard_normal((19, 23))
-            P[2, 3] = np.nan
+        for vd, (V, P, steps) in rc.member_loop_case().items():
             pg = init(V, 0.5, 5.0, randstate=np.random.RandomState(9))
             po = ora_bps.initialize_bps(V, 0.5, 5.0, randstate=np.random.RandomState(9))
             assert pg["eps_par"] == po["eps_par"] and pg["eps_perp"] == po["eps_perp"]
             assert _bits_equal(pg["V_par"], po["V_par"]) and _bits_equal(pg["V_perp"], po["V_perp"])
             dg = dr = None
-            for step in range(1, 4):
+            for step in steps:
                 h = V + gen(pg, step * 5.0)
                 assert isinstance(h, pysteps_b200.noise.motion.PerturbedVelocity)
                 out_g, dg = extrap(P, h, [1.0], displacement_prev=dg, return_displacement=True,
                                    allow_nonfinite_values=True, b200_resident=True)
                 assert isinstance(dg, _device.DeviceField) and dg.shape == (2, 19, 23)
-                out_r, dr = ref(P, V + ora_bps.generate_bps(po, step * 5.0), [1.0], displacement_prev=dr,
-                                return_displacement=True, allow_nonfinite_values=True)
+                out_r, dr = ora.extrapolate(P, V + ora_bps.generate_bps(po, step * 5.0), [1.0], displacement_prev=dr,
+                                            return_displacement=True, allow_nonfinite_values=True)
+                fp.assert_same(out_r, golden, f"member_loop/{vd}/{step}/out")
+                fp.assert_same(dr, golden, f"member_loop/{vd}/{step}/displacement")
                 assert _bits_equal(out_g, out_r) and _bits_equal(np.asarray(dg), dr)
             assert _bits_equal(np.asarray(V + gen(pg, 7.0)), V + ora_bps.generate_bps(po, 7.0))
         # non-finite perturbed field: the extrapolator's own check fires (semilagrangian.py:118-123)
@@ -173,14 +173,13 @@ def test_member_loop_with_handles_matches_reference_expression():
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_spline_orders_host_logic_and_kernel_bodies(seed, monkeypatch):
+def test_spline_orders_host_logic_and_kernel_bodies(seed, monkeypatch, golden):
     """interp_order 0, 2..5: the
     shim's branch -- trajectories per leadtime, prefilter, sampling, mask warps, outval="min" on
     the zero-filled copy, bands -- driven through the emulated C ABI, whose spline entry points
     are the CUDA kernels' own bodies compiled for the host (tests/host_kernels)."""
     import pysteps_b200
     extrap = pysteps_b200.extrapolation.semilagrangian.extrapolate
-    ref, live = _reference()
     rng = np.random.default_rng(300 + seed)
     with cpu_abi.emulated():
         with pytest.raises(RuntimeError, match="spline order not supported"):
@@ -189,11 +188,13 @@ def test_spline_orders_host_logic_and_kernel_bodies(seed, monkeypatch):
         for it in range(60):
             Pin, Vin, ts, outval, kw = _random_call(rng)
             kw["interp_order"] = int(rng.choice([0, 2, 3, 3, 4, 5]))
-            want, werr, wdep = _run(ref, Pin, Vin, ts, outval, kw)
+            want, werr, wdep = _run(ora.extrapolate, Pin, Vin, ts, outval, kw)
             got, gerr, gdep = _run(extrap, Pin, Vin, ts, outval, kw)
             ctx = f"seed {seed} case {it}: ts={ts!r} outval={outval!r} kw={ {k: (v.shape if isinstance(v, np.ndarray) else v) for k, v in kw.items()} }"
             if gerr is not None and "inf in precip" in gerr[1]:
                 continue
+            fp.assert_call(got, gerr, golden, f"spline/{seed}/{it}", ctx)
+            assert "\n".join(gdep) == golden[f"spline/{seed}/{it}/deprecations"], ctx
             assert gerr == werr and gdep == wdep, ctx
             if werr is not None:
                 continue

@@ -1,9 +1,10 @@
 """CPU test of the HOST logic of pysteps_b200.motion.vet (argument handling, error messages,
 padding / sector bookkeeping, indexing, intermediate steps, the SciPy optimiser loop) over
-randomised argument combinations -- against the oracle's restatement of vet.py and, when the
-reference's own extension has been built out of tree (tests/golden/gen_vet_golden.py,
-/tmp/vetbuild), against the live reference.  The three C-ABI entry points are emulated by the
-oracle (tests/cpu_abi.py): numerics here say nothing about the kernels."""
+randomised argument combinations -- against the oracle's restatement of vet.py and the
+reference's stored results and errors on the same calls (tests/golden/reference_host_golden.npz,
+written by tests/golden/gen_reference_golden.py with the reference's extension built with its own
+flags).  The three C-ABI entry points are emulated by the oracle (tests/cpu_abi.py): numerics here
+say nothing about the kernels."""
 import os
 import warnings
 
@@ -11,18 +12,14 @@ import numpy as np
 import pytest
 
 import cpu_abi
+import fingerprint as fp
 from oracle import vet as ora
 from pysteps_b200 import _synthetic as syn
 
 
-def _live_reference():
-    from _refimport import available, ref_module
-    if available() and os.path.isdir("/tmp/vetbuild/pysteps/motion"):
-        try:
-            return ref_module("pysteps.motion.vet", "/tmp/vetbuild").vet
-        except ImportError:
-            return None
-    return None
+@pytest.fixture(scope="module")
+def golden():
+    return fp.load(os.path.join(os.path.dirname(__file__), "golden", "reference_host_golden.npz"))
 
 
 def _random_call(rng):
@@ -77,9 +74,8 @@ def _run(fn, inp, kw):
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_vet_host_logic(seed):
+def test_vet_host_logic(seed, golden):
     from pysteps_b200.motion.vet import vet
-    live = _live_reference()
     rng = np.random.default_rng(700 + seed)
     n_err = n_ok = 0
     with cpu_abi.emulated():
@@ -89,9 +85,7 @@ def test_vet_host_logic(seed):
             want, werr = _run(ora.vet, inp, kw)
             ctx = f"seed {seed} case {it}: shape={inp.shape} kw={ {k: (v.shape if isinstance(v, np.ndarray) else v) for k, v in kw.items()} }"
             assert gerr == werr, ctx
-            if live is not None:
-                ref, rerr = _run(live, inp, kw)
-                assert gerr == rerr, ctx
+            assert fp._error_text(gerr) == golden[f"vet/{seed}/{it}/error"], ctx
             if gerr is not None:
                 n_err += 1
                 continue
@@ -101,12 +95,10 @@ def test_vet_host_logic(seed):
                 for a, b in zip(got[1], want[1]):
                     assert np.array_equal(np.asarray(a), np.asarray(b)), ctx
                 got, want = got[0], want[0]
-                if live is not None:
-                    ref = ref[0]
             # same cost / gradient evaluations and the same SciPy optimiser -> identical fields
             assert got.shape == want.shape and np.array_equal(got, want), ctx
-            if live is not None:      # the reference extension is built with -ffast-math
-                assert ref.shape == got.shape and np.abs(ref - got).max() < 1e-3, ctx
+            # the reference extension is built with -ffast-math
+            fp.assert_close(got, golden, f"vet/{seed}/{it}/field", 1e-3, ctx)
     assert n_err >= 3 and n_ok >= 10, (n_err, n_ok)
 
 

@@ -5,12 +5,15 @@ arithmetic and index logic of the spline kernels without a GPU; the device build
 in spelling every float64 operation as a round-to-nearest intrinsic."""
 import ctypes
 import math
+import os
 
 import numpy as np
 import pytest
-from conftest import assert_bits_equal
+from conftest import ROOT, assert_bits_equal
 
+import fingerprint as fp
 import host_kernels
+import reference_cases as rc
 from oracle import semilagrangian as ora
 
 POLES = {0: (), 2: (-0.171572875253809902396622551580603843,), 3: (-0.267949192431122706472553658494127633,),
@@ -19,6 +22,11 @@ POLES = {0: (), 2: (-0.171572875253809902396622551580603843,), 3: (-0.2679491924
 F32, F64 = 0, 1
 MODES = {"constant": 0, "nearest": 1}
 _dp = ctypes.POINTER(ctypes.c_double)
+
+
+@pytest.fixture(scope="module")
+def host_golden():
+    return fp.load(os.path.join(ROOT, "tests", "golden", "reference_host_golden.npz"))
 
 
 def _p(a):
@@ -230,63 +238,36 @@ def test_knn_pair_formulation_build_matches_scipy_ckdtree(kind, n):
             assert np.array_equal(d, want_d.reshape(len(queries), -1)), (kind, n, k, depth)
 
 
-def test_outlier_body_matches_the_reference_at_ties():
+def test_outlier_body_matches_the_reference_at_ties(host_golden):
     """detect_outliers of the reference (scipy cKDTree + np.cov + np.linalg.inv) on vector sets with
-    many equidistant and coincident positions: the body's flags equal the reference's (live when
-    /root/reference exists) and the oracle's in cKDTree mode."""
+    many equidistant and coincident positions: the body's flags equal the reference's stored ones
+    and the oracle's in cKDTree mode."""
     from oracle import lucaskanade as ora_lk
-    try:
-        from _refimport import available, ref_module
-        live = ref_module("pysteps.utils.cleansing").detect_outliers if available() else None
-    except Exception:  # noqa: BLE001
-        live = None
     L = host_kernels.lib()
     L.host_detect_outliers_ckdtree.restype = None
-    rng = np.random.default_rng(31)
-    for it in range(30):
-        n = int(rng.choice([2, 3, 10, 40, 300, 1500]))
-        xy = np.floor(rng.uniform(0, rng.choice([6, 30, 200]), (n, 2)))
-        if it % 3 == 0 and n >= 8:
-            xy[: n // 4] = xy[n // 4: 2 * (n // 4)]
-        uv = np.stack([2 + 0.3 * rng.standard_normal(n), -1 + 0.3 * rng.standard_normal(n)], 1)
-        uv[::7] += 2.0
-        k = int(rng.choice([5, 30, 100]))
-        thr = float(rng.choice([1, 2, 3]))
+    for it, (uv, xy, k, thr) in enumerate(rc.outlier_body_cases()):
+        n = len(xy)
         flags = np.empty(n, np.uint8)
         L.host_detect_outliers_ckdtree(_p(np.ascontiguousarray(uv)), _p(np.ascontiguousarray(xy)), n,
                                        ctypes.c_double(thr), k, _p(flags))
         with ora_lk.knn_mode("ckdtree"):
             want = ora_lk.detect_outliers(uv, thr, xy, k)
         assert np.array_equal(flags.astype(bool), want), (it, n, k, thr)
-        if live is not None and n >= 3:
-            import warnings
-            with warnings.catch_warnings():
-                warnings.simplefilter("ignore")
-                assert np.array_equal(flags.astype(bool), live(uv, thr, xy, k)), (it, n, k, thr)
+        if n >= 3:
+            ref = np.unpackbits(host_golden[f"outliers/{it}"], count=n).astype(bool)
+            assert np.array_equal(flags.astype(bool), ref), (it, n, k, thr)
 
 
-def test_exact_idw_body_matches_the_reference_at_every_grid_point():
+def test_exact_idw_body_matches_the_reference_at_every_grid_point(host_golden):
     """idwinterp2d with cKDTree's neighbour order, numpy's pairwise weight sum and in-order
-    accumulation (knn_body.cuh: idw_point): equal to the reference at ALL grid points, ties and
-    coincident vectors included, to the last bits of np.power vs pow."""
+    accumulation (knn_body.cuh: idw_point): equal to the oracle at ALL grid points and to the
+    reference's stored fields (bit for bit, or within 1e-14 on a stored sample), ties and coincident
+    vectors included, to the last bits of np.power vs pow."""
     from oracle import lucaskanade as ora_lk
-    try:
-        from _refimport import available, ref_module
-        live = ref_module("pysteps.utils.interpolate").idwinterp2d if available() else None
-    except Exception:  # noqa: BLE001
-        live = None
     L = host_kernels.lib()
     L.host_idw_fill_ckdtree.restype = None
-    rng = np.random.default_rng(2)
-    for it in range(14):
-        n = int(rng.choice([2, 30, 200, 800]))
-        W, H = int(rng.choice([40, 120])), int(rng.choice([30, 90]))
-        xy = np.floor(rng.uniform(0, max(W, H), (n, 2)) * 2) / 2
-        if it % 3 == 0 and n >= 8:
-            xy[: n // 4] = xy[n // 4: 2 * (n // 4)]
-        uv = np.ascontiguousarray(rng.standard_normal((n, 2)))
-        k = int(min(rng.choice([1, 4, 20, 30]), n))
-        power, off = float(rng.choice([0.5, 1.0, 2.0])), float(rng.choice([0.5, 1.0]))
+    for it, (xy, uv, W, H, k, power, off) in enumerate(rc.idw_body_cases()):
+        n = len(xy)
         xg, yg = np.arange(W, dtype=float), np.arange(H, dtype=float)
         out = np.empty((2, H, W))
         L.host_idw_fill_ckdtree(_p(np.ascontiguousarray(xy)), _p(uv), n, 2, k, ctypes.c_double(power),
@@ -294,9 +275,7 @@ def test_exact_idw_body_matches_the_reference_at_every_grid_point():
         with ora_lk.knn_mode("ckdtree"):
             want = ora_lk.idwinterp2d(xy, uv, np.arange(W), np.arange(H), power=power, k=k, dist_offset=off)
         assert np.abs(out - want).max() <= 1e-14, (it, n, k, power)
-        if live is not None:
-            ref = live(xy, uv, np.arange(W), np.arange(H), power=power, k=k, dist_offset=off)
-            assert np.abs(out - ref).max() <= 1e-14, (it, n, k, power)
+        fp.assert_close(out, host_golden, f"idw/{it}", 1e-14, f"case {it} {(n, k, power)}")
 
 
 @pytest.mark.parametrize("shape", [(17, 23), (5, 40), (1, 9), (3, 3), (64, 80)])

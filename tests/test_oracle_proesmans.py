@@ -6,11 +6,14 @@
     (-O3 -ffast-math, setup.py:27-28; tests/golden/gen_proesmans_golden.py): that build does not
     define its rounding, and the solver turns a flipped branch into a local change of up to a
     pixel, so only well-conditioned cases are compared closely;
-  * against both builds live when they are still present in this container."""
+  * against stored outputs of both builds on randomised calls
+    (tests/golden/reference_proesmans_golden.npz, tests/golden/gen_reference_golden.py)."""
 import os
 
+import fingerprint as fp
 import numpy as np
 import pytest
+import reference_cases as rc
 from conftest import assert_bits_equal
 
 from oracle import proesmans as ora
@@ -27,6 +30,11 @@ def golden():
 @pytest.fixture(scope="module")
 def strict_golden():
     return np.load(os.path.join(os.path.dirname(__file__), "golden", "proesmans_strict_golden.npz"))
+
+
+@pytest.fixture(scope="module")
+def random_golden():
+    return fp.load(os.path.join(os.path.dirname(__file__), "golden", "reference_proesmans_golden.npz"))
 
 
 @pytest.fixture
@@ -61,14 +69,12 @@ def test_oracle_matches_the_fastmath_build_of_the_reference(name, golden):
         assert np.abs(ref_adv).max() > 0.3   # the cases do exercise the solver
 
 
-def test_gaussian_prefilter_against_live_reference(raster_mean):
-    ref = _live("/tmp/proes_strict")
+def test_gaussian_prefilter_against_live_reference(raster_mean, random_golden):
     frames, _ = build_case("default_96x128")
-    for std in (0.8, 2.5):
-        a, qa = ref(frames, filter_std=std, num_iter=10, num_levels=3, full_output=True)
+    for std in rc.PROESMANS_PREFILTER_STDS:
         b, qb = ora.proesmans(frames, filter_std=std, num_iter=10, num_levels=3, full_output=True)
-        assert_bits_equal(b, a, f"filter_std {std}")
-        assert_bits_equal(qb, qa, f"filter_std {std} quality")
+        fp.assert_same(b, random_golden, f"proesmans_prefilter/{std}/advfield", f"filter_std {std}")
+        fp.assert_same(qb, random_golden, f"proesmans_prefilter/{std}/quality", f"filter_std {std} quality")
 
 
 def test_argument_errors():
@@ -78,65 +84,19 @@ def test_argument_errors():
         ora.proesmans(np.zeros((3, 8, 8)))
 
 
-def _live(build):
-    """The reference's proesmans() with the extension of `build`, the extension loaded straight
-    from its file so that both builds can live in one process."""
-    import glob
-    import importlib.util
-    from _refimport import available
-    hits = glob.glob(os.path.join(build, "pysteps", "motion", "_proesmans*.so"))
-    if not (available() and hits):
-        pytest.skip(f"reference extension not built in {build}")
-    try:
-        spec = importlib.util.spec_from_file_location("pysteps.motion._proesmans", hits[0])
-        ext = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ext)
-    except ImportError:
-        pytest.skip("reference extension not importable")
-
-    def proesmans(input_images, lam=50.0, num_iter=100, num_levels=6, filter_std=0.0, full_output=False):
-        # pysteps/motion/proesmans.py:73-94
-        from scipy.ndimage import gaussian_filter
-        im = np.stack([input_images[-2, :, :].copy(), input_images[-1, :, :].copy()])
-        im_min, im_max = np.min(im), np.max(im)
-        if im_max - im_min > 1e-8:
-            im = (im - im_min) / (im_max - im_min) * 255.0
-        if filter_std > 0.0:
-            im[0, :, :] = gaussian_filter(im[0, :, :], filter_std)
-            im[1, :, :] = gaussian_filter(im[1, :, :], filter_std)
-        advfield, quality = ext._compute_advection_field(im, lam, num_iter, num_levels)
-        return (advfield, quality) if full_output else advfield[0]
-
-    return proesmans
-
-
-def _random_cases(seed, count):
-    from pysteps_b200 import _synthetic as syn
-    rng = np.random.default_rng(seed)
-    for _ in range(count):
-        m, n = int(rng.integers(8, 160)), int(rng.integers(8, 160))
-        lv = int(rng.integers(1, 6))
-        if (m >> (lv - 1)) < 1 or (n >> (lv - 1)) < 1:
-            continue   # an empty pyramid level: the reference reads out of bounds there
-        fr = syn.rain_frames(m, n, 2, int(rng.integers(0, 100)), dx=int(rng.integers(-3, 4)), dy=int(rng.integers(-3, 4)))
-        yield fr, dict(lam=float(rng.choice([5.0, 50.0, 1000.0])), num_iter=int(rng.choice([1, 7, 30, 100])),
-                       num_levels=lv, full_output=True)
-
-
-def test_live_ieee_build_bitwise(raster_mean):
-    ref = _live("/tmp/proes_strict")
-    for fr, kw in _random_cases(21, 25):
-        a, qa = ref(fr, **kw)
+def test_live_ieee_build_bitwise(raster_mean, random_golden):
+    for i, (fr, kw) in enumerate(rc.proesmans_random_cases(21, 25)):
         b, qb = ora.proesmans(fr, **kw)
-        assert_bits_equal(b, a, f"{fr.shape} {kw}")
-        assert_bits_equal(qb, qa, f"{fr.shape} {kw} quality")
+        fp.assert_same(b, random_golden, f"proesmans_strict/{i}/advfield", f"{fr.shape} {kw}")
+        fp.assert_same(qb, random_golden, f"proesmans_strict/{i}/quality", f"{fr.shape} {kw} quality")
 
 
-def test_live_fastmath_build_statistically():
-    ref = _live("/tmp/vetbuild")
+def test_live_fastmath_build_statistically(random_golden):
+    """max deviation from the -ffast-math build, over the stored sample of each field"""
     devs = []
-    for fr, kw in _random_cases(22, 25):
-        a, _ = ref(fr, **kw)
+    for i, (fr, kw) in enumerate(rc.proesmans_random_cases(22, 25)):
         b, _ = ora.proesmans(fr, **kw)
-        devs.append(np.abs(a - b).max())
+        want = random_golden[f"proesmans_fast/{i}/advfield/sample"]
+        assert b.shape == fp.layout(random_golden, f"proesmans_fast/{i}/advfield")[1]
+        devs.append(np.abs(fp.sample(b, random_golden, f"proesmans_fast/{i}/advfield") - want).max())
     assert np.median(devs) < 1e-9, sorted(devs)

@@ -1,12 +1,14 @@
 """CPU tests: the spline part of the semi-Lagrangian oracle (oracle/spline_oracle.c --
 scipy.ndimage.map_coordinates for orders 0 and 2..5 with prefilter) is pinned bit for bit against
 the scipy binary; the extrapolator with interp_order 0 / 3 against the reference's stored
-outputs (tests/test_oracle_sl.py, SPLINE_CASES) and, when /root/reference exists, the live
-reference."""
+outputs (tests/test_oracle_sl.py, SPLINE_CASES) and on 60 randomised calls
+(tests/golden/reference_golden.npz)."""
 import warnings
 
+import fingerprint as fp
 import numpy as np
 import pytest
+import reference_cases as rc
 from conftest import assert_bits_equal
 from scipy import ndimage as ndi
 
@@ -63,41 +65,23 @@ def test_float32_input_rounds_like_scipy():
         assert_bits_equal(got, ref, mode)
 
 
-def test_extrapolate_spline_orders_against_live_reference():
-    from _refimport import available, ref_module
-    if not available():
-        pytest.skip("/root/reference not present (GPU box)")
-    ref = ref_module("pysteps.extrapolation.semilagrangian").extrapolate
-    rng = np.random.default_rng(77)
+def test_extrapolate_spline_orders_against_live_reference(reference_golden):
+    """60 small randomised calls (tests/golden/reference_cases.py) against the reference's stored
+    outputs and error messages, bit for bit."""
+    g = reference_golden
     warnings.simplefilter("ignore")
-    for it in range(60):
-        m, n = int(rng.integers(1, 30)), int(rng.integers(1, 30))
-        P = (rng.standard_normal((m, n)) * 5).astype(rng.choice([np.float64, np.float32]))
-        V = (rng.standard_normal((2, m, n)) * rng.choice([0.5, 3.0, 20.0])).astype(rng.choice([np.float64, np.float32]))
-        kw = {"interp_order": int(rng.choice([0, 2, 3, 3, 4, 5])), "map_coordinates_mode": str(rng.choice(["constant", "nearest"]))}
-        if rng.random() < 0.4:
-            P[rng.random((m, n)) < 0.2] = np.nan
-            kw["allow_nonfinite_values"] = True
-        if rng.random() < 0.4:
-            kw["n_iter"] = int(rng.integers(0, 4))
-        if rng.random() < 0.4:
-            kw["return_displacement"] = True
-        outval = rng.choice([np.nan, 0.0, -15.0]) if rng.random() < 0.8 else "min"
-        ts = int(rng.integers(1, 4)) if rng.random() < 0.5 else [0.5, 1.25]
-        try:
-            want, werr = ref(P.copy(), V.copy(), ts, outval, **kw), None
-        except ValueError as e:
-            want, werr = None, str(e)
+    for it, (P, V, ts, outval, kw) in enumerate(rc.spline_cases()):
+        werr = g.get(f"spline/{it}/error")
         try:
             got, gerr = ora.extrapolate(P.copy(), V.copy(), ts, outval, **kw), None
         except ValueError as e:
             got, gerr = None, str(e)
         assert gerr == werr, (it, kw)
         if werr is None:
-            for a, b in zip(got if isinstance(got, tuple) else (got,), want if isinstance(want, tuple) else (want,)):
-                assert_bits_equal(a, b, f"case {it} {kw}")
+            got = got if isinstance(got, tuple) else (got,)
+            assert f"spline/{it}/{len(got)}" not in g, (it, kw)
+            for j, a in enumerate(got):
+                fp.assert_same(a, g, f"spline/{it}/{j}", f"case {it} {kw}")
     with pytest.raises(RuntimeError) as e_ora:
         ora.extrapolate(np.ones((4, 4)), np.ones((2, 4, 4)), 1, interp_order=6)
-    with pytest.raises(RuntimeError) as e_ref:
-        ref(np.ones((4, 4)), np.ones((2, 4, 4)), 1, interp_order=6)
-    assert str(e_ora.value) == str(e_ref.value)
+    assert str(e_ora.value) == str(g["spline/order6_error"])

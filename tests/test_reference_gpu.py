@@ -1,17 +1,27 @@
-"""The REFERENCE ITSELF against the CUDA path, on the B200: pysteps v1.21.3 travels to the GPU box
-in compiled form (oracle/_ref, built by oracle/build_ref.py from /root/reference) and runs there
-unmodified -- stand-alone functions, the ensemble member loop and a whole nowcasts.steps forecast,
-once with its stock methods and once with the B200 methods registered over the stock names
-(pysteps_b200.register(override=True)), real kernels both times."""
+"""The CUDA path against pysteps v1.21.3 itself, on the B200.  Stand-alone functions are compared
+with the reference's stored outputs (tests/golden/reference_gpu_golden.npz, written by
+tests/golden/gen_reference_golden.py); the ensemble member loop and a whole nowcasts.steps forecast
+run the reference's own loop, once with its stock methods and once with the B200 methods registered
+over the stock names (pysteps_b200.register(override=True)), real kernels both times, and need the
+reference in compiled form (oracle/_ref, built by oracle/build_ref.py)."""
 import contextlib
 import io
+import os
 import warnings
 
+import fingerprint as fp
 import numpy as np
 import pytest
-from conftest import assert_bits_equal
+import reference_cases as rc
 
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture(scope="module")
+def golden():
+    import torch
+    assert torch.cuda.is_available(), "gpu-marked test needs a GPU"
+    return fp.load(os.path.join(os.path.dirname(__file__), "golden", "reference_gpu_golden.npz"))
 
 
 @pytest.fixture(scope="module")
@@ -20,7 +30,8 @@ def ref():
     assert torch.cuda.is_available(), "gpu-marked test needs a GPU"
     from oracle import refimport
     if not refimport.available(extensions=True):
-        pytest.skip("oracle/_ref has not been built (python oracle/build_ref.py where /root/reference exists)")
+        pytest.skip("the reference's own nowcast loop is needed: oracle/_ref has not been built "
+                    "(python oracle/build_ref.py with the pysteps v1.21.3 source tree)")
     return refimport
 
 
@@ -30,54 +41,37 @@ def _quiet(fn, *a, **k):
         return fn(*a, **k)
 
 
-@pytest.mark.parametrize("shape,nframes,seed", [((512, 512), 2, 0), ((512, 512), 3, 1), ((301, 417), 3, 2),
-                                                ((1024, 1024), 2, 3)])
-def test_dense_lucaskanade_equals_the_reference(ref, shape, nframes, seed):
+@pytest.mark.parametrize("shape,nframes,seed", rc.LK_GPU_CASES)
+def test_dense_lucaskanade_equals_the_reference(golden, shape, nframes, seed):
     import pysteps_b200
-    from pysteps_b200 import _synthetic as syn
-    rlk = ref.ref_module("pysteps.motion.lucaskanade").dense_lucaskanade
+    key = f"lk/{shape[0]}x{shape[1]}x{nframes}/{seed}"
     lk = pysteps_b200.motion.get_method("lk")
-    fr = syn.rain_frames(shape[0], shape[1], nframes, seed)
-    if seed == 2:
-        fr = np.stack([syn.nan_disc(f, 0.1) for f in fr])
-    rxy, ruv = _quiet(rlk, fr.copy(), dense=False)
+    fr = rc.lk_gpu_frames(shape, nframes, seed)
     xy, uv = lk(fr.copy(), dense=False)
-    assert np.array_equal(xy, rxy) and np.array_equal(uv, ruv), "sparse vectors"
-    V, Vr = lk(fr.copy()), _quiet(rlk, fr.copy())
-    assert V.shape == Vr.shape and V.dtype == Vr.dtype
-    assert np.abs(V - Vr).max() <= 1e-12, "dense field at every pixel"
+    fp.assert_same(xy, golden, key + "/xy", "sparse vectors")
+    fp.assert_same(uv, golden, key + "/uv", "sparse vectors")
+    V = lk(fr.copy())
+    fp.assert_close(V, golden, key + "/dense", 1e-12, "dense field")
+    # every pixel, against the oracle (tests/test_oracle_lk.py pins it to the reference's stored fields)
+    from oracle import lucaskanade as ora
+    assert np.abs(V - ora.dense_lucaskanade(fr.copy())).max() <= 1e-12, "dense field at every pixel"
 
 
 @pytest.mark.parametrize("case", range(6))
-def test_extrapolate_equals_the_reference(ref, case):
+def test_extrapolate_equals_the_reference(golden, case):
     import pysteps_b200
-    from pysteps_b200 import _synthetic as syn
-    rsl = ref.ref_module("pysteps.extrapolation.semilagrangian").extrapolate
     sl = pysteps_b200.extrapolation.get_method("semilagrangian")
-    m, n = ((256, 320), (511, 300), (128, 128), (400, 400), (200, 256), (333, 222))[case]
-    P = syn.rain_field(m, n, case)
-    V = syn.velocity_field(m, n, case, ("smooth", "rotation")[case % 2]) * (1.0 + case)
-    kw = [dict(), dict(n_iter=3), dict(outval="min"), dict(interp_order=3, map_coordinates_mode="nearest"),
-          dict(allow_nonfinite_values=True), dict(interp_order=0)][case]
-    if case == 4:
-        P = syn.nan_disc(P)
-    ts = [4, 3, [0.5, 1.0, 2.5], 2, 3, 3][case]
-    want, wd = rsl(P, V, ts, return_displacement=True, **kw)
+    P, V, ts, kw = rc.sl_gpu_case(case)
     got, gd = sl(P, V, ts, return_displacement=True, **kw)
-    assert_bits_equal(got, want, f"case {case} fields")
-    assert_bits_equal(gd, wd, f"case {case} displacement")
+    fp.assert_same(got, golden, f"sl/{case}/fields", f"case {case} fields")
+    fp.assert_same(gd, golden, f"sl/{case}/displacement", f"case {case} displacement")
 
 
-def test_vet_close_to_the_reference_build(ref):
+def test_vet_close_to_the_reference_build(golden):
     """the reference extension is built with -ffast-math (setup.py:27-28): 1e-6 px"""
     import pysteps_b200
-    from pysteps_b200 import _synthetic as syn
-    rvet = ref.ref_module("pysteps.motion.vet").vet
     vet = pysteps_b200.motion.get_method("vet")
-    fr = syn.rain_frames(256, 256, 2, 3)
-    want = rvet(fr, verbose=False)
-    got = vet(fr, verbose=False)
-    assert got.shape == want.shape and np.abs(got - want).max() < 1e-6
+    fp.assert_close(vet(rc.vet_gpu_frames(), verbose=False), golden, "vet/field", 1e-6)
 
 
 def test_steps_forecast_with_registered_b200_methods(ref):
